@@ -74,7 +74,34 @@ def parse():
                          "(own process group), reported as sub-objects of the chain line; delta / pagerank (single-GPU kernels with "
                          "per-kernel rooflines and parity) at N = 1 only; '' or 'none' = skip")
     ap.add_argument("--side-timeout", type=int, default=300, help="seconds a side workload may take before its children are stopped")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="chain workload, b200 arm: after the timed steps write rank 0's result of the last timed step to DIR as "
+                         "float64 .npy files (row_ptr, and a fixed seeded sample of col_idx with its positions) so that two builds "
+                         "can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.workload != "chain"):
+        ap.error("--dump-outputs is implemented for the chain workload's b200 arm only")
+    return a
+
+
+DUMP_SAMPLE = 1 << 21          # column indices kept from a larger result: 2 x 16 MB of float64 with their positions
+
+
+def dump_outputs(out_dir, F):
+    """Write the CSR a caller of the chain receives -- row pointers in full, column indices as a sample at positions drawn
+    with a fixed seed -- as float64 (exact: every value is below 2^53)."""
+    p, j, _ = F.export_csr()
+    nnz = len(j)
+    if nnz > DUMP_SAMPLE:
+        pos = np.sort(np.random.default_rng(12345).choice(nnz, size=DUMP_SAMPLE, replace=False))
+    else:
+        pos = np.arange(nnz)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "row_ptr.npy"), p.astype(np.float64))
+    np.save(os.path.join(out_dir, "col_idx_sample.npy"), j[pos].astype(np.float64))
+    np.save(os.path.join(out_dir, "col_idx_sample_pos.npy"), pos.astype(np.float64))
 
 
 def peaks():
@@ -414,10 +441,13 @@ def run_b200(a):
     e0.record(stream)
     flops = 0
     nnz_out = 0
+    last = None
     for i in range(a.warmup, nb):
         F = F0[i].dup()
         flops += chain(F, tally=True)
         nnz_out += F.nvals()
+        if a.dump_outputs and rank == 0 and i == nb - 1:
+            last = F                  # outlives the timed window only when it is to be written out
         del F
     e1.record(stream)
     barrier()
@@ -431,6 +461,9 @@ def run_b200(a):
         if L.B200_kernel_stats(name.encode(), C.byref(m), C.byref(nl), C.byref(by)) == 0 and nl.value:
             kstats[name] = {"ms": m.value, "launches": nl.value, "bytes": by.value}
     fb.set_option("timing", 0)
+    if last is not None:
+        dump_outputs(a.dump_outputs, last)
+        del last
 
     # ---- e2e arm: host buffers in, host CSR out, through the public C ABI ----
     # the CSR hand-off needs 4 B per result entry of pinned host memory (6-7 GB at 512 sources): only where it is timed

@@ -1,14 +1,15 @@
 #!/usr/bin/env python
 """Regenerates tests/golden/reference_ffi_symbols.json: every GraphBLAS / LAGraph C symbol the reference's wrapper layer
 links against.  A symbol counts when (a) graph/src/graph/graphblas/mod.rs (bindgen) or lagraph*_bindings.rs declares it as an
-`extern "C"` function or static and (b) one of the wrapper files below names it outside a comment.  Run in the build
-container (needs /root/reference); the JSON is what tests/test_abi.py checks `nm -D libb200grb.so` against everywhere."""
+`extern "C"` function or static and (b) one of the wrapper files below names it outside a comment.  Needs a checkout of the
+reference: python tests/golden/make_ffi_symbols.py <reference checkout>.  The JSON is what tests/test_abi.py checks
+`nm -D libb200grb.so` against."""
 import json
 import os
 import re
 import sys
 
-REF = "/root/reference"
+REF = None                  # the reference checkout, from the command line
 GB = "graph/src/graph/graphblas"
 WRAPPERS = [f"{GB}/matrix.rs", f"{GB}/vector.rs", f"{GB}/tensor.rs", f"{GB}/versioned_matrix.rs"]
 # the traversal operators and the BFS procedure reach the C API through the wrappers plus these direct call sites
@@ -46,6 +47,10 @@ def used(rel):
 
 
 def main():
+    global REF
+    if len(sys.argv) != 2:
+        return "usage: python tests/golden/make_ffi_symbols.py <reference checkout>"
+    REF = sys.argv[1]
     fn, st = declared()
     functions, statics = {}, {}
     for rel in WRAPPERS + CALLERS:
